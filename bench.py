@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — images/sec of the Uformer-B 256x256 forward (BASELINE.json configs[1]) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--mode fwd|train]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--mode fwd|train] [--dump-outputs DIR]
 
 `--mode train` (not the default; BASELINE configs[2]) times the data-parallel training step instead: batch 8 per GPU,
 native forward + recompute backward + NCCL bucketed gradient all-reduce + native AdamW (uformer_b200.training).
@@ -18,6 +18,10 @@ the public API with pinned HOST input, H2D copy and D2H of the restored image in
 in an extra instrumented step.  `cpu_baseline` / `--impl reference` time the CPU oracle port of the
 reference forward (oracle/lewin_oracle.py; the reference itself is Python and cannot travel to the
 GPU box) on the host cores, on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step of rank 0 computed as DIR/<name>.npy (float32): the restored images
+(`restored`, fwd) or the loss (`loss`, train).  Inputs and weights are seeded, so two builds run with the same arguments can be
+compared output for output.  An output over the 64 MB budget is replaced by a fixed, seeded sample of its elements.
 """
 import argparse
 import json
@@ -36,6 +40,7 @@ import torch  # noqa: E402
 UFORMER_B = dict(img_size=256, embed_dim=32, win_size=8, token_projection="linear", token_mlp="leff",
                  depths=[1, 2, 8, 8, 2, 8, 8, 2, 1], modulator=True, dd_in=3)       # utils/model_utils.py:76-78
 GFLOP_PER_IMG = 173.1          # BASELINE.md §2 (2 x 86.57 GMAC)
+DUMP_BYTES = 64 << 20          # --dump-outputs budget over all arrays
 
 
 def note(msg):
@@ -85,6 +90,21 @@ class ClockSampler:
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         reasons = [n for i, n in enumerate(names) if any(len(r) > 2 + i and r[2 + i] == "Active" for r in self.rows)]
         return dict(sm_mhz=sm[len(sm) // 2] if sm else None, sm_max_mhz=max(mx) if mx else None, reasons=reasons, samples=len(sm))
+
+
+def dump_outputs(outdir, arrays):
+    """Each tensor of `arrays` -> outdir/<name>.npy as float32; one larger than its share of DUMP_BYTES becomes the same
+    seeded random sample of its elements (sorted flat indices) on every run."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    cap = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(outdir, name + ".npy"), a.numpy())
+    note(f"outputs of the last timed step written to {outdir}: {', '.join(arrays)}")
 
 
 def build_engine(device, seed=1234):
@@ -146,7 +166,7 @@ def run_reference_arm(args, rank, world):
     nimg = 4                         # bounded sample of the batch-32 step
     fwd = _cpu_forward_fn(nimg)
     threads = _pick_threads(fwd)     # doubles as warm-up
-    steps, warm = max(1, min(args.steps, 5)), 1
+    steps, warm = args.steps, 1
     t0 = time.perf_counter()
     for _ in range(steps):
         fwd()
@@ -195,7 +215,7 @@ def run_reference_train(args, rank):
         torch.sqrt((out - clean) ** 2 + 1e-6).mean().backward()
         opt.step()
     step()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         step()
@@ -241,18 +261,19 @@ def run_train(args, rank, world, local):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(total device ms over `steps` steps, max over ranks; what the last step returned)"""
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
         for s, e in evs:
             flush.zero_()
             s.record()
-            fn()
+            out = fn()
             e.record()
         barrier()
         t = torch.tensor([sum(s.elapsed_time(e) for s, e in evs)], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return t.item()
+        return t.item(), out
 
     def step_dev():
         return step(noisy_d, clean_d)
@@ -272,9 +293,11 @@ def run_train(args, rank, world, local):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    total_ms = timed(step_dev, args.steps)
+    total_ms, loss = timed(step_dev, args.steps)
     clocks = sampler.stop() if rank == 0 else None
-    e2e_ms = timed(step_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss})
+    e2e_ms, _ = timed(step_e2e, args.steps)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -315,7 +338,13 @@ def main():
                          "512x512 images in one whole-image forward, default batch 8)")
     ap.add_argument("--residual", default=None, choices=["auto", "fp32", "bf16"],
                     help="residual-stream precision between the kernels of a stage (default: the engine's default, fp32)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy, float32, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the native engine's outputs (--impl ours)")
     if args.residual:
         os.environ["UFORMER_B200_RESIDUAL"] = args.residual
     rank = int(os.environ.get("RANK", 0))
@@ -363,19 +392,20 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(total device ms over `steps` steps, max over ranks; what the last step returned)"""
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
         for s, e in evs:
             flush.zero_()                    # L2 flush, outside the event bracket
             s.record()
-            fn()
+            out = fn()
             e.record()
         barrier()
         ms = sum(s.elapsed_time(e) for s, e in evs)
         t = torch.tensor([ms], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return t.item()
+        return t.item(), out
 
     # device-resident leg: the forward captured once into a CUDA graph (uformer_b200.GraphedForward) and replayed;
     # falls back to eager launches if capture is unavailable
@@ -444,9 +474,11 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    total_ms = timed(step_dev, args.steps)
+    total_ms, restored = timed(step_dev, args.steps)
     launches = launches_per_step * args.steps                  # the graph replays exactly these launches every step
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"restored": restored})   # before later forwards can reuse any buffer
     note(f"device-resident: {total_ms / args.steps:.2f} ms/step; timing e2e (host buffers)")
     run_e2e(2)
     e2e_ms = run_e2e(args.steps)

@@ -37,6 +37,18 @@ def rel_max(a, b):
     return ((a.double() - b.double()).abs().max() / b.double().abs().max().clamp_min(1e-30)).item()
 
 
+def rel_l2_sampled(t, ref):
+    """rel-L2 of `t` against a stored sample of a reference tensor (dict(stride, sample, norm), see
+    golden/make_reference_checks.py): the larger of the error over the sample and the relative difference of the norms."""
+    t = t.detach()
+    return max(rel_l2(t.reshape(-1)[::ref["stride"]], ref["sample"]), abs(float(t.double().norm()) - ref["norm"]) / ref["norm"])
+
+
+def max_err_sampled(t, ref):
+    """max |t - ref| over a stored sample of a reference tensor, relative to the full reference tensor's max |ref|."""
+    return float((t.detach().reshape(-1)[::ref["stride"]].double() - ref["sample"].double()).abs().max()) / ref["absmax"]
+
+
 def state_checksum(state):
     s = 0.0
     for k in sorted(state):

@@ -182,6 +182,33 @@ def test_bench_reference_arm_contract():
     assert d["e2e"] == {"value": d["value"], "unit": "img/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float32 .npy per output, whole while it fits the budget; past it, the same seeded sample of
+    its elements on every run, and all arrays together within the budget."""
+    import numpy as np
+    import bench
+    t = torch.randn(4, 3, 8, 8).to(torch.bfloat16)
+    bench.dump_outputs(str(tmp_path / "a"), {"restored": t})
+    a = np.load(tmp_path / "a" / "restored.npy")
+    assert a.dtype == np.float32 and a.shape == (4, 3, 8, 8) and np.array_equal(a, t.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 400)
+    big = torch.randn(1000)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"restored": big, "loss": torch.tensor(0.5)})
+    b, c = np.load(tmp_path / "b" / "restored.npy"), np.load(tmp_path / "c" / "restored.npy")
+    assert b.dtype == np.float32 and b.shape == (50,) and np.array_equal(b, c) and np.isin(b, big.numpy()).all()
+    assert np.load(tmp_path / "b" / "loss.npy") == np.float32(0.5)
+    assert sum(f.stat().st_size - 128 for f in (tmp_path / "b").iterdir()) <= 400          # .npy header: 128 bytes
+
+
+def test_bench_steps_argument():
+    """--steps is the number of timed steps; zero or fewer is refused before anything runs."""
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=300)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="uses fake device pointers: only meaningful (and safe) where no launch can happen")
 def test_alignment_validation_without_gpu():
     """Pointers the kernels access with 16-byte vectors / bulk copies must be 16-byte aligned: rejected with LW_ERR_ALIGN

@@ -1,8 +1,8 @@
 """CPU: the training path's host logic and backward math.
 
 * uformer_b200/restated.py (the statements backward differentiates) against the golden gradients generated from the
-  unmodified reference (tests/golden/make_train_golden.py), and live against the reference's own autograd — incl.
-  training-mode stochastic depth with a shared RNG seed — whenever /root/reference is mounted;
+  unmodified reference (tests/golden/make_train_golden.py), and against the reference's own autograd on single blocks and
+  samplers — incl. training-mode stochastic depth with a shared RNG seed (tests/golden/make_reference_checks.py);
 * autograd.NativeFn wiring (recompute-from-input backward) with a stand-in forward;
 * FlatArena layout, in-place gradient accumulation, bucket construction.
 No native compute runs here (no GPU): the modules' forward still raises EngineUnavailable on CPU.
@@ -14,9 +14,8 @@ import uformer_b200 as U
 from uformer_b200 import autograd as AG
 from uformer_b200 import restated as R
 from uformer_b200 import training as T
-from helpers import load_golden, rel_l2
+from helpers import load_golden, rel_l2, rel_l2_sampled, state_checksum
 from paramgen import randomize_state
-from refshim import reference_available, import_reference_model
 
 
 def _charbonnier(x, y, eps=1e-3):
@@ -48,58 +47,49 @@ def test_restated_backward_matches_reference_golden():
     print("worst sampled-gradient rel-L2 vs reference:", worst)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted")
 @pytest.mark.parametrize("dim,heads,H,shift,modu,dp", [(32, 1, 16, 0, False, 0.0), (64, 2, 24, 4, True, 0.3), (32, 2, 16, 4, True, 0.5)])
 def test_restated_block_vs_reference_autograd(dim, heads, H, shift, modu, dp):
     """Forward, input gradient and every parameter gradient of one LeWin block, training mode, stochastic depth drawn
-    from the same RNG state on both sides (model.py:986-987)."""
-    m = import_reference_model()
-    ref = m.LeWinTransformerBlock(dim, (H, H), heads, win_size=8, shift_size=shift, modulator=modu, drop_path=dp)
+    from the same RNG state as the reference's (model.py:986-987)."""
+    c = next(c for c in load_golden("reference_checks")["block_autograd"] if c["case"][:6] == (dim, heads, H, shift, modu, dp))
+    xseed = c["case"][6]
     ours = U.LeWinTransformerBlock(dim, (H, H), heads, win_size=8, shift_size=shift, modulator=modu, drop_path=dp)
-    st = randomize_state(ref.state_dict(), 21)
-    ref.load_state_dict(st)
+    st = randomize_state(ours.state_dict(), 21)
+    assert abs(state_checksum(st) - c["checksum"]) <= 1e-6 * c["checksum"]
     ours.load_state_dict(st, strict=True)
-    ref.train()
     ours.train()
     B = 4
-    x = torch.randn(B, H * H, dim)
-    xr = x.clone().requires_grad_(True)
-    xo = x.clone().requires_grad_(True)
-    gout = torch.randn(B, H * H, dim)
+    gen = torch.Generator().manual_seed(xseed)
+    xo = torch.randn(B, H * H, dim, generator=gen).requires_grad_(True)
+    gout = torch.randn(B, H * H, dim, generator=gen)
     torch.manual_seed(99)
-    yr = ref(xr)
-    yr.backward(gout)
-    torch.manual_seed(99)
-    s1 = ours.drop_path.draw(B, x.device) if dp > 0 else None
-    s2 = ours.drop_path.draw(B, x.device) if dp > 0 else None
+    s1 = ours.drop_path.draw(B, xo.device) if dp > 0 else None
+    s2 = ours.drop_path.draw(B, xo.device) if dp > 0 else None
     yo = R.lewin_block(ours, xo, None, s1, s2)
     yo.backward(gout)
-    assert rel_l2(yo.detach(), yr.detach()) < 1e-5
-    assert rel_l2(xo.grad, xr.grad) < 1e-4
-    pr = dict(ref.named_parameters())
+    assert rel_l2_sampled(yo, c["y"]) < 1e-5
+    assert rel_l2_sampled(xo.grad, c["dx"]) < 1e-4
+    assert set(c["grads"]) == {k for k, _ in ours.named_parameters()}
     for k, p in ours.named_parameters():
-        assert rel_l2(p.grad, pr[k].grad) < 1e-4, k
+        assert rel_l2_sampled(p.grad, c["grads"][k]) < 1e-4, k
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted")
 def test_restated_samplers_vs_reference_autograd():
-    m = import_reference_model()
-    for ref, ours, fn, shape in [(m.Downsample(16, 32), U.Downsample(16, 32), R.downsample, (2, 256, 16)),
-                                 (m.Upsample(32, 8), U.Upsample(32, 8), R.upsample, (2, 64, 32)),
-                                 (m.LeFF(16, 64), U.LeFF(16, 64), R.leff, (2, 256, 16))]:
-        st = randomize_state(ref.state_dict(), 3)
-        ref.load_state_dict(st)
+    checks = load_golden("reference_checks")["samplers"]
+    for name, ours, fn in [("down", U.Downsample(16, 32), R.downsample), ("up", U.Upsample(32, 8), R.upsample),
+                           ("leff", U.LeFF(16, 64), R.leff)]:
+        c = checks[name]
+        st = randomize_state(ours.state_dict(), 3)
+        assert abs(state_checksum(st) - c["checksum"]) <= 1e-6 * c["checksum"], name
         ours.load_state_dict(st, strict=True)
-        x = torch.randn(*shape)
-        xr, xo = x.clone().requires_grad_(True), x.clone().requires_grad_(True)
-        yr, yo = ref(xr), fn(ours, xo)
-        g = torch.randn_like(yr)
-        yr.backward(g)
-        yo.backward(g)
-        assert rel_l2(yo.detach(), yr.detach()) < 1e-5 and rel_l2(xo.grad, xr.grad) < 1e-4
-        pr = dict(ref.named_parameters())
+        gen = torch.Generator().manual_seed(c["seed"])
+        xo = torch.randn(*c["shape"], generator=gen).requires_grad_(True)
+        yo = fn(ours, xo)
+        yo.backward(torch.randn(yo.shape, generator=gen))
+        assert rel_l2_sampled(yo, c["y"]) < 1e-5 and rel_l2_sampled(xo.grad, c["dx"]) < 1e-4, name
+        assert set(c["grads"]) == {k for k, _ in ours.named_parameters()}, name
         for k, p in ours.named_parameters():
-            assert rel_l2(p.grad, pr[k].grad) < 1e-4, k
+            assert rel_l2_sampled(p.grad, c["grads"][k]) < 1e-4, (name, k)
 
 
 def test_nativefn_recompute_backward_wiring():
@@ -183,21 +173,13 @@ def test_training_ops_have_no_cpu_path():
         net(torch.rand(1, 3, 128, 128))
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted")
 def test_stochastic_depth_schedule_and_flops_equal_reference():
     """Per-block drop_path rates (model.py:1093-1095 and the decoder slices :1170-1232) and Uformer.flops() of the engine's
     own caller equal the reference's for the Uformer-B configuration."""
-    import contextlib
-    import io
-    m = import_reference_model()
-    cfg = dict(img_size=256, embed_dim=32, win_size=8, token_projection="linear", token_mlp="leff", depths=[1, 2, 8, 8, 2, 8, 8, 2, 1],
-               modulator=True, dd_in=3, drop_path_rate=0.1)
-    r, o = m.Uformer(**cfg), U.Uformer(**cfg)
+    c = load_golden("reference_checks")["uformer_b"]
+    o = U.Uformer(**c["cfg"])
     stages = ["encoderlayer_0", "encoderlayer_1", "encoderlayer_2", "encoderlayer_3", "conv", "decoderlayer_0", "decoderlayer_1",
               "decoderlayer_2", "decoderlayer_3"]
-
-    def rates(net):
-        return [round(getattr(b.drop_path, "drop_prob", 0.0), 7) for n in stages for b in getattr(net, n).blocks]
-    assert rates(r) == rates(o) and max(rates(o)) == 0.1
-    with contextlib.redirect_stdout(io.StringIO()):                 # the reference prints per-layer GFLOPs
-        assert r.flops() == o.flops()
+    rates = [round(getattr(b.drop_path, "drop_prob", 0.0), 7) for n in stages for b in getattr(o, n).blocks]
+    assert rates == c["drop_path_rates"] and max(rates) == 0.1
+    assert o.flops() == c["flops"]
